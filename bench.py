@@ -85,9 +85,10 @@ def make_workload(workdir, ref_mbp, n_reads, read_len, seed, rank=0, paired=Fals
         t0 = time.time()
         contigs = gen_data.random_contigs(n_contigs, contig_len, 7)
         if ref_mbp <= 60:
-            # small enough for the reference's own `bwa index` (about a minute at most)
+            # small enough for the index builder on the CPU (the files of `bwa index`, byte for byte; 60 Mbp: 20 s, 3.8 GB on 8 cores)
+            import bwa_b200.index_build as ib
             gen_data.write_fasta(fa, contigs)
-            subprocess.run([REF_BWA, "index", fa], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            ib.build(fa, device="cpu", verbose=False)
         else:
             # `bwa index` needs hours at this size (bwa.1:767): same files from the GPU builder (bwa_b200/index_build.py,
             # byte-identical to `bwa index` where both can run, see tests/test_gpu_parity.py::test_index_builder)
@@ -196,6 +197,38 @@ def time_reference(fa, fqs, n_sample, threads, keep_sam=False, mem_args=()):
     if n == 0 or real <= 0:
         raise RuntimeError("reference run produced no timing lines:\n" + r.stderr[-2000:])
     return n / real, n
+
+
+def dump_outputs(out_dir, sam, n_reads, fa, n_sample=262144):
+    """What one mem_process_seqs call returned -- the SAM text of each read -- as arrays DIR/<name>.npy (float64, one row per
+    read of a fixed sample of at most n_sample reads, seed 0): fields of the read's first record, its record count and the CRC-32
+    of its whole text, so that two builds can be compared output for output.  sam: char *[n_reads] (bb_batch_detach_sam)."""
+    import ctypes as C
+    import zlib
+    import numpy as np
+    rows = np.arange(n_reads) if n_reads <= n_sample else np.sort(np.random.default_rng(0).choice(n_reads, n_sample, replace=False))
+    names = open(fa + ".ann").read().split("\n")[1::2]
+    contig = {l.split()[1]: float(i) for i, l in enumerate(names) if l.strip()}
+    p = C.cast(sam, C.POINTER(C.c_char_p))
+    cols = {k: np.full(len(rows), -1.0) for k in ("flag", "ref_id", "pos", "mapq", "tlen", "as", "xs", "nm", "n_records", "sam_crc32")}
+    for j, i in enumerate(rows):
+        text = p[int(i)] or b""
+        rec = text.split(b"\n")
+        f = rec[0].split(b"\t")
+        cols["n_records"][j] = sum(1 for r in rec if r)
+        cols["sam_crc32"][j] = zlib.crc32(text)
+        if len(f) < 11:
+            continue
+        cols["flag"][j], cols["pos"][j], cols["mapq"][j], cols["tlen"][j] = int(f[1]), int(f[3]), int(f[4]), int(f[8])
+        cols["ref_id"][j] = contig.get(f[2].decode(), -1.0)
+        for t in f[11:]:
+            if t[:5] in (b"AS:i:", b"XS:i:", b"NM:i:"):
+                cols[t[:2].decode().lower()][j] = int(t[5:])
+    cols["read_index"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in cols.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    log("[bench] outputs of the last timed step (%d of %d reads) written to %s" % (len(rows), n_reads, out_dir))
 
 
 def supervise(argv):
@@ -324,6 +357,7 @@ def main():
     ap.add_argument("--inflight", type=int, default=int(os.environ.get("BWA_B200_INFLIGHT", "3")), help="mem_process_seqs calls issued at a time (host threads), as bwa-b200 mem does")
     ap.add_argument("--worker", action="store_true", help="(internal) run the measurement in this process; without it a parent process supervises the run")
     ap.add_argument("--dense-sa", type=int, default=int(os.environ.get("BWA_B200_DENSE_SA", "0")))
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="write what the last timed step returned (per-read SAM fields of a fixed sample) as DIR/<name>.npy")
     a = ap.parse_args()
     a.cpu_sample_given = a.cpu_sample is not None
     if a.cpu_sample is None:
@@ -510,6 +544,8 @@ def main():
         dist.barrier()
     clocks = sampler.stop()
     st = idx.stats()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, held[-1], n_reads, fa)   # held[-1]: the SAM of the step that completed last
     release()
     # Kernel-only figures (value, roofline): the timed region above overlaps several chunks on different streams, so
     # per-kernel event times there include waiting for each other.  Two more passes with ONE lane and ONE chunk give
@@ -606,10 +642,9 @@ def main():
                     cut = lambda l: b"\t".join(l.split(b"\t")[:9] + l.split(b"\t")[11:]).decode("latin1")[:600]
                     line["cpu_baseline"]["sam_diff"] = {"rc": rc, "lines_reference": len(la), "lines_b200": len(lb), "differing_lines": sum(1 for x, y in zip(la, lb) if x != y), "first_at": k,
                                                         "reference": cut(la[k]) if k < len(la) else None, "b200": cut(lb[k]) if k < len(lb) else None}
-                    keep = os.path.join(ROOT, "gpurun_out")
-                    if os.path.isdir(keep):
-                        import shutil
-                        shutil.copy(ref_out, os.path.join(keep, "sam_diff_reference.sam")); shutil.copy(mine, os.path.join(keep, "sam_diff_b200.sam"))
+                    import shutil
+                    shutil.copy(ref_out, os.path.join(a.workdir, "sam_diff_reference.sam")); shutil.copy(mine, os.path.join(a.workdir, "sam_diff_b200.sam"))
+                    line["cpu_baseline"]["sam_diff"]["kept"] = a.workdir
                 for f in (mine, ref_out):
                     os.remove(f)
                 if not mem_args and a.ref_mbp >= 1000:

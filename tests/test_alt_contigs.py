@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 import bwa_b200
-from conftest import CUSIMBIN, REF_BWA, ref_sam, run_sam
+from conftest import CUSIMBIN, index, md5, ref_sam_md5, run_sam
 
 
 def _make(tmp_path):
@@ -25,7 +25,7 @@ def _make(tmp_path):
     with open(fa, "wb") as f:
         for name, seq in ((b"chr1", base), (b"dup", other[:4000]), (b"chr1_alt", alt), (b"dup", other[4000:])):
             f.write(b">" + name + b"\n" + seq.tobytes() + b"\n")
-    subprocess.run([REF_BWA, "index", fa], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    index(fa)
     with open(fa + ".alt", "w") as f:
         f.write("@comment line\nchr1_alt\t0\t*\ndup\nchr1")      # last line unterminated: not an ALT contig
     contigs = [base, alt, other]
@@ -41,9 +41,9 @@ def _make(tmp_path):
 def _check(binary, tmp_path):
     fa, fqs, se = _make(tmp_path)
     for args in (["-K", "100000000", "-t", "3", fa] + fqs, ["-K", "100000000", "-t", "3", fa, se], ["-K", "100000000", "-t", "3", "-a", fa, se]):
-        want = ref_sam(args)
-        assert run_sam(binary, args) == want
-        assert b"pa:f:" in want or b"XA:Z:" in want or len(args) == 7
+        got = run_sam(binary, args)
+        assert md5(got) == ref_sam_md5(args)
+        assert b"pa:f:" in got or b"XA:Z:" in got or len(args) == 7
 
 
 def test_alt_contigs_emulated(built, tmp_path):

@@ -6,7 +6,7 @@ import subprocess
 
 import pytest
 
-from conftest import ROOT, ref_sam, strip_pg
+from conftest import ROOT, md5, ref_sam_md5, strip_pg
 
 ASAN_BIN = os.path.join(ROOT, "tests", "_build", "bwa-b200-cusim-asan")
 RUNS = [
@@ -35,4 +35,4 @@ def test_emulated_kernels_under_asan(data, asan_bin, name, ref, kw, extra, env):
     p = subprocess.run([asan_bin, "mem", "-v", "1"] + args, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=900)
     assert b"AddressSanitizer" not in p.stderr, p.stderr.decode()[-3000:]
     assert p.returncode == 0, p.stderr.decode()[-2000:]
-    assert strip_pg(p.stdout) == ref_sam(args)
+    assert md5(strip_pg(p.stdout)) == ref_sam_md5(args)

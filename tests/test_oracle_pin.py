@@ -1,7 +1,7 @@
 """Pins the CPU oracle (oracle/oracle_*.c) to the UNMODIFIED reference:
   * committed known-answer vectors produced by oracle/_ref/katdump (tests/golden/*.kat.gz, make_golden.sh);
-  * live katdump runs of the reference's FM-index functions on a generated index;
-  * whole-program SAM: host glue + oracle stages (tests/_build/bwa-b200-oracle) vs `oracle/_ref/bwa mem`.
+  * katdump runs of the reference's FM-index functions on a generated index (stored: tests/golden/katdump_*.txt.gz);
+  * whole-program SAM: host glue + oracle stages (tests/_build/bwa-b200-oracle) vs the md5 of `oracle/_ref/bwa mem`'s.
 No GPU needed."""
 import ctypes as C
 import gzip
@@ -12,7 +12,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import KATDUMP, ORACLE_SO, REF_BWA, ROOT, TESTBIN, md5, ref_sam, run_sam
+from conftest import ORACLE_SO, ROOT, TESTBIN, md5, ref_run, ref_sam_md5, run_sam
 
 CODE = {c: i for i, c in enumerate("ACGTN")}
 
@@ -114,7 +114,7 @@ def test_fm_index_live(orc, data):
     L = bwa_b200.lib()
     idx = L.bwa_idx_load(fa.encode(), 1)
     bwt = idx.contents.bwt
-    txt = subprocess.run([KATDUMP, "smem", fa, fq, "25"], stdout=subprocess.PIPE, check=True).stdout.decode().split("\n")
+    txt = ref_run("katdump", ["smem", fa, fq, "25"], "raw", keep="katdump_smem.txt.gz")["out"].decode().split("\n")
     seq, mem, one, n_checked = None, IntvV(), Intv(), 0
     reads = {}
     name = None
@@ -143,7 +143,7 @@ def test_fm_index_live(orc, data):
             assert (r, "%d,%d,%d,%d" % (one.x0, one.x1, one.x2, one.info)) == (ret, f[3]), l[:100]
     assert n_checked > 5000
     idx2 = L.bwa_idx_load(fa.encode(), 1)
-    for l in subprocess.run([KATDUMP, "sa", fa, "3000", "99"], stdout=subprocess.PIPE, check=True).stdout.decode().split("\n"):
+    for l in ref_run("katdump", ["sa", fa, "3000", "99"], "raw", keep="katdump_sa.txt.gz")["out"].decode().split("\n"):
         f = l.split()
         if f:
             assert orc.orc_sa(C.c_void_p(idx2.contents.bwt), C.c_uint64(int(f[1])), None) == int(f[2])
@@ -166,8 +166,8 @@ def test_host_glue_sam_vs_reference(data, name, ref, kw, extra):
     reference's output itself matches the committed md5 (pins the generators and the oracle build)."""
     fa, fqs = data.reads(ref, **kw)
     args = extra + ["-K", "100000000", "-t", "4", fa] + fqs
-    want = ref_sam(args)
+    want = ref_sam_md5(args)
     got = run_sam(TESTBIN, args)
-    assert got == want
+    assert md5(got) == want
     pins = json.load(open(os.path.join(ROOT, "tests/golden/sam_md5.json")))
-    assert pins[name] == md5(want), "reference SAM changed: regenerate tests/golden/sam_md5.json deliberately"
+    assert pins[name] == want, "reference SAM changed: regenerate tests/golden/sam_md5.json deliberately"

@@ -8,7 +8,7 @@ import subprocess
 
 import pytest
 
-from conftest import ROOT, ref_sam, strip_pg
+from conftest import ROOT, md5, ref_sam_md5, strip_pg
 
 TSAN_BIN = os.path.join(ROOT, "tests", "_build", "bwa-b200-tsan")
 
@@ -22,7 +22,7 @@ def test_host_pipeline_is_race_free(data):
     env = dict(os.environ, BWA_B200_INFLIGHT="3", BWA_B200_LANES="2", BWA_B200_CHUNK="16", TSAN_OPTIONS="halt_on_error=0 exitcode=0")
     p = subprocess.run([TSAN_BIN, "mem", "-v", "1"] + args, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=800)
     assert p.returncode == 0, p.stderr.decode()[-2000:]
-    assert strip_pg(p.stdout) == ref_sam(args)
+    assert md5(strip_pg(p.stdout)) == ref_sam_md5(args)
     reports = re.split(r"WARNING: ThreadSanitizer", p.stderr.decode())[1:]
     ours = []
     for rep in reports:

@@ -10,7 +10,7 @@ import subprocess
 import pytest
 
 import bwa_b200
-from conftest import CUSIMBIN, ref_sam, run_sam, strip_pg
+from conftest import CUSIMBIN, md5, ref_sam_md5, run_sam, strip_pg
 
 
 def _counts(binary, args, env=None):
@@ -30,14 +30,14 @@ def _check(binary, data, n_c1, n_stress):
     fa, fqs = data.reads("c1", tag="tl_pe%d" % n_c1, n=n_c1, seed=31, paired=True)
     args = ["-K", "100000000", "-t", "4", "-R", "@RG\\tID:grp1\\tSM:x", fa] + fqs
     sam, took, handed, lane = _counts(binary, args)
-    assert sam == ref_sam(args)
+    assert md5(sam) == ref_sam_md5(args)
     assert took == 2 * n_c1 and handed * 50 <= took and lane
     # repeat-rich reference, chimeric reads: many reads are handed back, the merged output is still the reference's
     for paired in (True, False):
         fa, fqs = data.reads("stress", tag=("tl_pe%d" if paired else "tl_se%d") % n_stress, n=n_stress, seed=32, paired=paired, err=(0.016, 0.002, 0.002), chimeric=0.05)
         args = ["-K", "100000000", "-t", "4", "-C", fa] + fqs
         sam, took, handed, lane = _counts(binary, args)
-        assert sam == ref_sam(args)
+        assert md5(sam) == ref_sam_md5(args)
         assert took >= n_stress and 0 < handed < took
         if paired:
             assert _counts.sw > 0          # mate rescue ran its local alignments on the device (K6)
@@ -52,7 +52,7 @@ def _check(binary, data, n_c1, n_stress):
     for extra, on in ((["-a"], False), (["-5"], False), (["-M", "-Y"], True), (["-P"], True), (["-S"], True), (["-T", "60", "-U", "9"], True)):
         args = extra + ["-K", "100000000", "-t", "4", fa] + fqs
         sam, took, handed, lane = _counts(binary, args)
-        assert sam == ref_sam(args), extra
+        assert md5(sam) == ref_sam_md5(args), extra
         assert (took > 0) == on, extra
 
 
@@ -76,7 +76,7 @@ def test_device_tail_fasta_input_and_several_chunks(data, tmp_path, monkeypatch)
     args = ["-K", "100000000", "-t", "3", fa] + fas
     monkeypatch.setenv("BWA_B200_CHUNK", "64")
     monkeypatch.setenv("BWA_B200_LANES", "2")
-    assert run_sam(CUSIMBIN, args) == ref_sam(args)
+    assert md5(run_sam(CUSIMBIN, args)) == ref_sam_md5(args)
 
 
 @pytest.mark.gpu
@@ -93,7 +93,7 @@ def _sb16(binary, data):
     for kw in (dict(tag="sb_se", n=400, seed=41), dict(tag="sb_pe", n=200, seed=42, paired=True)):
         fa, fqs = data.reads("c1", **kw)
         args = ["-K", "100000000", "-t", "4", fa] + fqs
-        assert run_sam(binary, args) == ref_sam(args)
+        assert md5(run_sam(binary, args)) == ref_sam_md5(args)
 
 
 def test_small_superblocks_emulated(data):
@@ -117,7 +117,7 @@ def _check_seed_filter(binary, data, n_1k, n_pb, pb_len):
         args = extra + ["-K", "100000000", "-t", "4", fa] + fqs
         sam, _, _, _ = _counts(binary, args)
         assert _counts.sw > 0, (ref, kw)
-        assert sam == ref_sam(args), (ref, kw)
+        assert md5(sam) == ref_sam_md5(args), (ref, kw)
         s2, _, _, _ = _counts(binary, args, {"BWA_B200_DEVICE_SEEDSW": "0"})
         assert _counts.sw == 0 and s2 == sam
 

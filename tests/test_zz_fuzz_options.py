@@ -8,7 +8,7 @@ import subprocess
 import pytest
 
 import bwa_b200
-from conftest import CUSIMBIN, REF_BWA, strip_pg
+from conftest import CUSIMBIN, md5, ref_run, strip_pg
 from fuzz_cases import command
 
 # BWA_B200_FUZZ_FROM/TO widen the emulated sweep (e.g. 10..300 after a kernel change); the default keeps the CPU suite short
@@ -19,11 +19,11 @@ GPU_CASES = list(range(0, 24)) + [114]
 
 
 def _both(binary, args):
-    r = subprocess.run([REF_BWA, "mem", "-v", "1"] + args, stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=600)
+    r = ref_run("bwa", ["mem", "-v", "1"] + args)
     g = subprocess.run([binary, "mem", "-v", "1"] + args, stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=600)
-    assert (r.returncode == 0) == (g.returncode == 0), g.stderr.decode()[-2000:]
-    if r.returncode == 0:
-        assert strip_pg(g.stdout) == strip_pg(r.stdout)
+    assert (r["rc"] == 0) == (g.returncode == 0), g.stderr.decode()[-2000:]
+    if r["rc"] == 0:
+        assert md5(strip_pg(g.stdout)) == r["md5"]
 
 
 @pytest.mark.parametrize("k", CPU_CASES)
